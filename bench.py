@@ -2,6 +2,7 @@
 """bench.py -- throughput of the quorum-tally + Reed-Solomon accept path on B200.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg3|cfg2|cfg3b|cfg4|cfg5]
+                  [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic input.  Default workload (cfg3,
 BASELINE.json configs[2], the configuration the north-star target is quoted on): the fused RSPaxos accept
@@ -72,7 +73,15 @@ def parse_args():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-sub", action="store_true", help="skip the cfg2/cfg3b/cfg4/cfg5 sub-benches")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="cfg3 / cfg2: after the timed steps, write what the last timed step computed (a seeded sample of the "
+                         "groups: parity planes, commit words, commit_bar) to DIR/<name>.npy, so that two builds can be compared")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload not in ("cfg3", "cfg2")):
+        ap.error("--dump-outputs covers the GPU arm's cfg3 and cfg2 steps")
+    return args
 
 
 def measured_peaks():
@@ -274,7 +283,7 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    r = cpu_arm(max(5, args.steps), max(1, args.warmup), args.groups, args.workload)
+    r = cpu_arm(args.steps, max(1, args.warmup), args.groups, args.workload)
     value = r["gbs"] if args.workload != "cfg2" else r["slots_per_s"]
     unit = "GB/s" if args.workload != "cfg2" else "slots/s"
     line = {
@@ -329,6 +338,31 @@ def _time_steps(torch, fn, steps, warmup):
     return a.elapsed_time(b) / steps
 
 
+DUMP_BYTES = 60_000_000     # --dump-outputs stays under 64 MB
+DUMP_SEED = 0x5EED0D
+
+
+def dump_step_outputs(torch, dev, out_dir, parity, committed, bar, n, L):
+    """Writes what one accept step returned, for a fixed seeded sample of its n groups, as float arrays:
+    groups (the sampled group indices), parity (P, k, L) shard bytes, commit_words (k, 2) low / high 32 bits of each
+    commit bitmap, commit_bar (k,).  parity is None when the step did not encode, committed / bar when it did not tally."""
+    per_group = (parity.shape[0] * L * 4 if parity is not None else 0) + (24 if committed is not None else 0) + 8
+    k = min(n, DUMP_BYTES // per_group)
+    idx = np.arange(n) if k == n else np.sort(np.random.default_rng(DUMP_SEED).choice(n, k, replace=False))
+    idx_t = torch.from_numpy(idx).to(dev)
+    out = {"groups": idx.astype(np.float64)}
+    if parity is not None:
+        out["parity"] = parity[:, idx_t, :L].cpu().numpy().astype(np.float32)
+    if committed is not None:
+        cw = committed[idx_t].cpu().numpy().view(np.uint64)
+        out["commit_words"] = np.stack([cw & np.uint64(0xFFFFFFFF), cw >> np.uint64(32)], axis=1).astype(np.float64)
+        out["commit_bar"] = bar[idx_t].cpu().numpy().view(np.uint32).astype(np.float64)
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, a in out.items():
+        np.save(d / f"{name}.npy", a)
+
+
 def _max_over_ranks(torch, dist, dev, world, *vals):
     if world == 1:
         return vals if len(vals) > 1 else vals[0]
@@ -352,6 +386,8 @@ def run_ours(args):
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
     assert torch.cuda.is_available(), "bench.py needs a GPU (no CPU fallback)"
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs needs a single process (--gpus 1)")
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
     if world > 1:
@@ -483,6 +519,9 @@ def run_ours(args):
     clocks = sampler.stop() if sampler else None
     status = ctx.device_status()
     assert status == 0, f"device status {status}: a step-flag wait timed out"
+    if args.dump_outputs:                            # before the passes below launch the kernels again
+        dump_step_outputs(torch, dev, args.dump_outputs, parity if args.workload != "cfg2" else None,
+                          committed if (args.workload == "cfg2" or not args.no_tally) else None, bar, n, L)
     # kernel-only duration (CUDA events around the launches), measured in a second pass so the events do not perturb
     # the whole-step timing above
     k_evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.steps)]
