@@ -455,6 +455,44 @@ int ss_reconstruct_serve_dev(ss_ctx *ctx, const uint8_t *shard_planes, uint64_t 
                              const uint32_t *req_held, const uint32_t *req_excl, const uint8_t *req_status,
                              const uint64_t *reply_off, uint64_t n_requests, uint32_t *reply_mask, uint8_t *out);
 
+/* Reconstruct replies, receiving side (SURVEY 8f-4; handle_msg_reconstruct_reply, crossword/messages.rs:634-722,
+ * rspaxos/messages.rs:519-594), batched over a follower's window of instances.  Instance row r = g*window + s (group g,
+ * window slot s, window <= 64); its shard j sits at shard_planes + j*plane_stride + r*shard_stride in 16-byte aligned
+ * slots of capacity round_up(L,16), L = ceil(data_len/d) -- the geometry of ss_rs_reconstruct_uniform_dev.
+ * inst_status[r]: Status in declaration order (0 Null .. 2 Accepting, 3 Committed, 4 Executed); inst_bal[r]: Instance.bal;
+ * present[r] (in/out): bit j = shard j held (avail_shards_map); exec_bar[g] (in/out): the handler's commit_bar, relative
+ * to the window.  Reply i has the layout ss_reconstruct_serve_dev writes: the shards of reply_mask[i] in index order, one
+ * round_up(L,16)-byte slot each, at reply_buf + reply_off[i] (16-byte aligned offsets), so serve's output on one GPU,
+ * copied or read over NVLink, is this call's input on another.  reply_inst[i] = row of the instance, 0xffffffff (or any
+ * row >= n_groups*window) for a slot below start_slot or outside the window: skipped (crossword/messages.rs:641-643);
+ * reply_ballot[i] = the replier's ballot.  Three kernels on the context's stream:
+ *   absorb  reply i is taken when inst_status < Executed && reply_ballot >= inst_bal (crossword/messages.rs:667,
+ *           rspaxos/messages.rs:542; as in the release build, Accepting instances are absorbed too).  absorb_other
+ *           (rscoding.rs:296-345) fills empty slots only: every shard missing from present is claimed by exactly one reply
+ *           (atomicOr on present[r]) and its whole padded slot is copied; taken[i] (may be NULL) = the bits reply i won.
+ *           A mask with bits >= d+p is malformed network input: the reply is dropped whole (taken 0).
+ *   walk    per group from exec_bar[g]: advance while s < window, status >= Committed and popcount(present) >= d
+ *           (crossword/messages.rs:670-688, rspaxos/messages.rs:545-560).  submit[g] bit s = instance s passed (written for
+ *           every group); passed instances with fewer than d data shards are marked for decode and their present gains the
+ *           data bits.
+ *   decode  reconstruct_data of the marked rows (ss_rs_reconstruct_uniform_dev's kernels; RS(3,2) gets its row kernel).
+ * Not done here: setting Executed (the reference does it only for an empty ReqBatch, which takes the payload -- a host
+ * decision) and bincode ReconstructReply frames.
+ * Batched vs per-message: the reference walks only when a reply lands exactly on commit_bar, decoding at that moment;
+ * this call absorbs the whole batch, walks once, then decodes.  The end states (present, exec_bar, submit, data bytes)
+ * are the same when (1) on entry the instance at each bar is not ready (not both Committed and holding >= d shards) --
+ * the walk leaves every bar in that state, so it holds from call to call -- and (2) every reply for a slot at a ballot
+ * >= inst.bal carries shards of the same codeword, which Paxos safety gives for committed instances.  Which of several
+ * replies carrying the same missing shard wins it (taken) is unspecified.
+ * Errors: SS_ERR_INVALID_ARG for null buffers, window 0 or > 64, n_groups 0, data_len 0, misaligned planes / reply_buf /
+ * strides, shard_stride < round_up(L,16); SS_ERR_UNSUPPORTED when d+p > 12.  n_replies == 0: SS_OK, nothing launched and
+ * no output written. */
+int ss_reconstruct_reply_dev(ss_rs_coder *coder, uint8_t *shard_planes, uint64_t plane_stride, uint64_t shard_stride,
+                             uint32_t data_len, uint64_t n_groups, uint32_t window, const uint8_t *inst_status,
+                             const uint64_t *inst_bal, uint32_t *present, uint32_t *exec_bar, const uint8_t *reply_buf,
+                             const uint64_t *reply_off, const uint32_t *reply_mask, const uint32_t *reply_inst,
+                             const uint64_t *reply_ballot, uint64_t n_replies, uint64_t *submit, uint32_t *taken);
+
 /* Crossword follower gossip planning (SURVEY 8f-4; crossword/gossiping.rs:35-84 gossip_targets_excl) for
  * n_instances committed-but-incomplete instances of replica `me`: walking peers me+1, me+2, ... (mod population) and
  * skipping the instance's source peer (src_peer[i]) and peers absent from `peer_alive`, a peer is selected when its

@@ -100,6 +100,8 @@ SIGNATURES = {
     "ss_accept_reply_parse_dev": (_i, [_vp, _vp, _u64, _vp, _vp, _vp, _vp, _u64, _u64, _u32, _i, _vp, _vp, _vp, _vp, _vp]),
     "ss_wal_commit_pack_dev": (_i, [_vp, _vp, _vp, _u64, _u32, _vp, _vp, _vp, _u64, _vp]),
     "ss_reconstruct_serve_dev": (_i, [_vp, _vp, _u64, _u64, _u32, _u32, _vp, _vp, _vp, _vp, _vp, _u64, _vp, _vp]),
+    "ss_reconstruct_reply_dev": (_i, [_vp, _vp, _u64, _u64, _u32, _u64, _u32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                      _u64, _vp, _vp]),
     "ss_engine_create": (_i, [_vp, _vp, _u64, C.POINTER(_vp)]),
     "ss_engine_destroy": (_i, [_vp]),
     "ss_engine_view_get": (_i, [_vp, _vp]),

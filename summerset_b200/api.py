@@ -509,6 +509,32 @@ class ReedSolomon:
                                                      1 if data_only else 0, _ptr(status)))
         return status
 
+    def reconstruct_reply(self, shards: torch.Tensor, data_len: int, window: int, inst_status: torch.Tensor,
+                          inst_bal: torch.Tensor, present: torch.Tensor, exec_bar: torch.Tensor, reply_buf: torch.Tensor,
+                          reply_off: torch.Tensor, reply_mask: torch.Tensor, reply_inst: torch.Tensor,
+                          reply_ballot: torch.Tensor, want_taken: bool = True):
+        """ReconstructReply receiving for G groups of `window` instances (ss_reconstruct_reply_dev).  shards uint8
+        [d+p, G*window, shard_stride] (padded-16 slots), inst_status uint8 / inst_bal int64 / present int32 [G*window],
+        exec_bar int32 [G]; present and exec_bar are updated in place.  Replies in the layout reconstruct_serve writes:
+        reply_buf uint8, reply_off int64, reply_mask int32, reply_inst int32 (-1 = skip), reply_ballot int64.
+        Returns (submit int64 [G], taken int32 [R] or None)."""
+        assert shards.is_cuda and shards.dtype == torch.uint8 and shards.is_contiguous() and shards.dim() == 3
+        t, n, ss = shards.shape
+        assert t == self.d + self.p and n % window == 0
+        assert inst_status.dtype == torch.uint8 and inst_bal.dtype == torch.int64 and present.dtype == torch.int32
+        assert exec_bar.dtype == torch.int32 and reply_buf.dtype == torch.uint8 and reply_off.dtype == torch.int64
+        assert reply_mask.dtype == torch.int32 and reply_inst.dtype == torch.int32 and reply_ballot.dtype == torch.int64
+        G, R = n // window, reply_off.numel()
+        assert present.numel() == n and inst_status.numel() == n and inst_bal.numel() == n and exec_bar.numel() == G
+        # the call writes every entry of both, except that an empty batch launches nothing
+        submit = (torch.empty if R else torch.zeros)(G, dtype=torch.int64, device=shards.device)
+        taken = torch.empty(R, dtype=torch.int32, device=shards.device) if want_taken else None
+        check(self.lib.ss_reconstruct_reply_dev(self.h, _ptr(shards), n * ss, ss, data_len, G, window, _ptr(inst_status),
+                                                _ptr(inst_bal), _ptr(present), _ptr(exec_bar), _ptr(reply_buf),
+                                                _ptr(reply_off), _ptr(reply_mask), _ptr(reply_inst), _ptr(reply_ballot),
+                                                R, _ptr(submit), _ptr(taken)))
+        return submit, taken
+
     def accept_step_fused(self, data: torch.Tensor, data_len: int, parity: torch.Tensor, planes: torch.Tensor,
                           threshold: int, committed: torch.Tensor, commit_bar: Optional[torch.Tensor]) -> None:
         """BASELINE config 3 step: RS-encode n groups' request batches + tally their ack windows, one launch."""

@@ -12,6 +12,10 @@
 //   wal_commit_pack_kernel      newly committed instances -> WalEntry::CommitSlot{slot} records (rspaxos/mod.rs:231)
 //   reconstruct_serve_kernel    Reconstruct serving: reply shards = held & flip(exclude) per requested instance, packed
 //                               (crossword/messages.rs:577-632, rspaxos/messages.rs:468-517)
+//   reconstruct_absorb_kernel   ReconstructReply receiving: the replied shards a row lacks, claimed with atomicOr on its
+//   reconstruct_walk_kernel     present mask and copied into the shard planes; then the execution-bar walk per group
+//                               (crossword/messages.rs:634-722, rspaxos/messages.rs:519-594); reconstruct_data of the
+//                               walked rows runs through the uniform reconstruct kernels
 //
 // bincode 2 standard config facts are from knowledge of the crate (unpinned against the reference, DESIGN.md section 4);
 // every kernel is tested byte for byte against oracle/ss_wire.c.
@@ -303,6 +307,127 @@ __global__ void __launch_bounds__(kWireThreads) reconstruct_serve_kernel(const _
     }
 }
 
+struct AbsorbArgs {
+    uint8_t *planes;
+    uint64_t plane_stride, shard_stride;
+    uint32_t all, vpc;                  // all: the T shard bits; vpc: 16-byte vectors per padded shard slot
+    uint64_t n_rows;
+    const uint8_t *inst_status;
+    const uint64_t *inst_bal;
+    uint32_t *present;
+    const uint8_t *buf;
+    const uint64_t *reply_off;
+    const uint32_t *reply_mask, *reply_inst;
+    const uint64_t *reply_ballot;
+    uint64_t n;
+    uint32_t *taken;                    // may be null
+};
+
+// a warp per reply: handle_msg_reconstruct_reply's filter (crossword/messages.rs:667, rspaxos/messages.rs:542), then
+// absorb_other (rscoding.rs:336-342): only shards the row does not hold yet are written.  The atomicOr on present[r]
+// hands every missing slot to exactly one reply, so two replies' bytes never mix in a slot.
+__global__ void __launch_bounds__(kWireThreads) reconstruct_absorb_kernel(const __grid_constant__ AbsorbArgs A) {
+    const uint32_t lane = threadIdx.x & 31u;
+    const uint64_t warp = (static_cast<uint64_t>(blockIdx.x) * kWireThreads + threadIdx.x) >> 5;
+    const uint64_t nwarps = (static_cast<uint64_t>(gridDim.x) * kWireThreads) >> 5;
+    for (uint64_t i = warp; i < A.n; i += nwarps) {
+        uint32_t won = 0u, m = 0u, r = 0u;
+        if (lane == 0u) {
+            r = __ldg(A.reply_inst + i);
+            m = __ldg(A.reply_mask + i);
+            // r out of range (0xffffffff: slot < start_slot or beyond the window, messages.rs:641-643) and masks naming
+            // shards >= T (malformed) are dropped whole
+            if (r < A.n_rows && (m & ~A.all) == 0u && __ldg(A.inst_status + r) < 4u &&      // Status::Executed
+                __ldg(A.reply_ballot + i) >= __ldg(A.inst_bal + r))
+                won = m & ~atomicOr(A.present + r, m);
+            if (A.taken != nullptr) A.taken[i] = won;
+        }
+        won = __shfl_sync(0xffffffffu, won, 0);
+        if (won == 0u) continue;
+        m = __shfl_sync(0xffffffffu, m, 0);
+        r = __shfl_sync(0xffffffffu, r, 0);
+        const uint64_t slot_bytes = static_cast<uint64_t>(A.vpc) * 16u;
+        const uint8_t *src0 = A.buf + __ldg(A.reply_off + i);
+        uint8_t *dst0 = A.planes + static_cast<uint64_t>(r) * A.shard_stride;
+        while (won) {
+            const uint32_t j = static_cast<uint32_t>(__ffs(won) - 1);
+            won &= won - 1u;
+            // the reply carries its shards in index order, one padded slot each (the layout reconstruct_serve_kernel writes)
+            const uint8_t *src = src0 + static_cast<uint64_t>(__popc(m & ((1u << j) - 1u))) * slot_bytes;
+            uint8_t *dst = dst0 + static_cast<uint64_t>(j) * A.plane_stride;
+            // four loads in flight per lane before their stores: one at a time leaves HBM latency exposed
+            for (uint32_t base = 0; base < A.vpc; base += 128u) {
+                uint4 x[4];
+#pragma unroll
+                for (uint32_t k = 0; k < 4u; ++k) {
+                    const uint32_t v = base + lane + 32u * k;
+                    if (v < A.vpc) x[k] = dev::ldg128(src + v * 16u);
+                }
+#pragma unroll
+                for (uint32_t k = 0; k < 4u; ++k) {
+                    const uint32_t v = base + lane + 32u * k;
+                    if (v < A.vpc) dev::stg128_cs(dst + v * 16u, x[k]);
+                }
+            }
+        }
+    }
+}
+
+struct WalkArgs {
+    const uint8_t *inst_status;
+    uint32_t *present;
+    uint32_t *exec_bar;
+    uint64_t *submit;
+    uint32_t *dec_present;              // [n_rows] present mask the decode kernel sees: all ones = intact, nothing to do
+    uint64_t G;
+    uint32_t W, d, all, dmask;
+};
+
+// a warp per group, two window slots per lane: the execution-bar walk of handle_msg_reconstruct_reply
+// (crossword/messages.rs:670-688, rspaxos/messages.rs:545-560) once over the absorbed state
+__global__ void __launch_bounds__(kWireThreads) reconstruct_walk_kernel(const __grid_constant__ WalkArgs A) {
+    const uint32_t lane = threadIdx.x & 31u;
+    const uint64_t warp = (static_cast<uint64_t>(blockIdx.x) * kWireThreads + threadIdx.x) >> 5;
+    const uint64_t nwarps = (static_cast<uint64_t>(gridDim.x) * kWireThreads) >> 5;
+    for (uint64_t g = warp; g < A.G; g += nwarps) {
+        const uint64_t row0 = g * A.W;
+        uint32_t pm[2] = {0u, 0u};
+        bool ready[2] = {false, false};
+#pragma unroll
+        for (uint32_t h = 0; h < 2u; ++h) {
+            const uint32_t s = lane + 32u * h;
+            if (s < A.W) {
+                pm[h] = A.present[row0 + s];
+                // status >= Committed and avail_shards() >= d
+                ready[h] = __ldg(A.inst_status + row0 + s) >= 3u && static_cast<uint32_t>(__popc(pm[h] & A.all)) >= A.d;
+            }
+        }
+        const uint64_t rdy = static_cast<uint64_t>(__ballot_sync(0xffffffffu, ready[0])) |
+                             (static_cast<uint64_t>(__ballot_sync(0xffffffffu, ready[1])) << 32);
+        const uint32_t bar = A.exec_bar[g];
+        uint64_t pass = 0ull;
+        uint32_t len = 0u;
+        if (bar < A.W) {
+            const uint64_t x = ~(rdy >> bar);          // slots >= W are never ready, so the run ends inside the window
+            len = x ? static_cast<uint32_t>(__ffsll(static_cast<long long>(x)) - 1) : 64u;
+            pass = (len >= 64u ? ~0ull : ((1ull << len) - 1ull)) << bar;
+        }
+#pragma unroll
+        for (uint32_t h = 0; h < 2u; ++h) {
+            const uint32_t s = lane + 32u * h;
+            if (s >= A.W) continue;
+            // passed with fewer than d data shards: reconstruct_data, after which the row holds every data shard
+            const bool decode = ((pass >> s) & 1ull) && (pm[h] & A.dmask) != A.dmask;
+            A.dec_present[row0 + s] = decode ? (pm[h] & A.all) : 0xffffffffu;
+            if (decode) A.present[row0 + s] = pm[h] | A.dmask;
+        }
+        if (lane == 0u) {
+            A.submit[g] = pass;
+            A.exec_bar[g] = bar + len;
+        }
+    }
+}
+
 static inline uint32_t wire_grid(ss_ctx *ctx, uint64_t items, uint32_t per_cta) {
     uint64_t ctas = (items + per_cta - 1) / per_cta;
     const uint64_t cap = static_cast<uint64_t>(ctx->sm_count) * 8ull * 8ull;
@@ -410,6 +535,59 @@ int ss_reconstruct_serve_dev(ss_ctx *ctx, const uint8_t *shard_planes, uint64_t 
     SS_CUDA(cudaGetLastError());
     ctx->launches++;
     return SS_OK;
+}
+
+int ss_reconstruct_reply_dev(ss_rs_coder *coder, uint8_t *shard_planes, uint64_t plane_stride, uint64_t shard_stride,
+                             uint32_t data_len, uint64_t n_groups, uint32_t window, const uint8_t *inst_status,
+                             const uint64_t *inst_bal, uint32_t *present, uint32_t *exec_bar, const uint8_t *reply_buf,
+                             const uint64_t *reply_off, const uint32_t *reply_mask, const uint32_t *reply_inst,
+                             const uint64_t *reply_ballot, uint64_t n_replies, uint64_t *submit, uint32_t *taken) {
+    if (coder == nullptr) return set_error(SS_ERR_INVALID_ARG, "null coder");
+    ss_ctx *ctx = coder->ctx;
+    SS_TRY(ctx_bind(ctx));
+    if (n_replies == 0) return SS_OK;
+    if (!shard_planes || !inst_status || !inst_bal || !present || !exec_bar || !reply_buf || !reply_off || !reply_mask ||
+        !reply_inst || !reply_ballot || !submit)
+        return set_error(SS_ERR_INVALID_ARG, "null buffer");
+    if (window == 0 || window > 64) return set_error(SS_ERR_INVALID_ARG, "window must be 1..64 instances");
+    // row indices are u32 with 0xffffffff reserved for "no instance"
+    if (n_groups == 0 || n_groups > 0xfffffffeull / window) return set_error(SS_ERR_INVALID_ARG, "n_groups * window must be 1..2^32-2");
+    if (data_len == 0) return set_error(SS_ERR_INVALID_ARG, "null codewords cannot be reconstructed (rscoding.rs:495-497)");
+    if (!coder->batch_ok || !coder->dec_ok)
+        return set_error(SS_ERR_UNSUPPORTED, "batched reconstruct needs d+p <= 12 (coder is %d,%d)", coder->d, coder->p);
+    const uint32_t d = static_cast<uint32_t>(coder->d), T = d + static_cast<uint32_t>(coder->p);
+    const uint32_t L = (data_len + d - 1u) / d, vpc = (L + 15u) >> 4;
+    if (((reinterpret_cast<uintptr_t>(shard_planes) | reinterpret_cast<uintptr_t>(reply_buf) | plane_stride | shard_stride) & 15u) ||
+        shard_stride < static_cast<uint64_t>(vpc) * 16u)
+        return set_error(SS_ERR_INVALID_ARG, "reconstruct replies need 16-byte aligned, padded shard slots (shard_stride >= round_up(L,16))");
+    const uint64_t n = n_groups * window;
+    // scratch: [0, keep) stays free for launch_rs_reconstruct_uniform's own offsets (n*12 + 256 bytes for codes other than
+    // RS(3,2)); then the decode kernel's present masks and its per-row status, which nobody reads
+    const uint64_t keep = (n * 12u + 256u + 255u) & ~uint64_t(255);
+    void *scr = nullptr;
+    SS_TRY(ctx_scratch(ctx, keep + n * 8u, &scr));
+    uint32_t *dec_present = reinterpret_cast<uint32_t *>(static_cast<uint8_t *>(scr) + keep);
+    int32_t *dec_status = reinterpret_cast<int32_t *>(dec_present + n);
+
+    AbsorbArgs A;
+    A.planes = shard_planes; A.plane_stride = plane_stride; A.shard_stride = shard_stride;
+    A.all = (1u << T) - 1u; A.vpc = vpc; A.n_rows = n;
+    A.inst_status = inst_status; A.inst_bal = inst_bal; A.present = present;
+    A.buf = reply_buf; A.reply_off = reply_off; A.reply_mask = reply_mask; A.reply_inst = reply_inst; A.reply_ballot = reply_ballot;
+    A.n = n_replies; A.taken = taken;
+    reconstruct_absorb_kernel<<<wire_grid(ctx, n_replies, kWireThreads / 32), kWireThreads, 0, ctx->stream>>>(A);
+    SS_CUDA(cudaGetLastError());
+    ctx->launches++;
+
+    WalkArgs W;
+    W.inst_status = inst_status; W.present = present; W.exec_bar = exec_bar; W.submit = submit; W.dec_present = dec_present;
+    W.G = n_groups; W.W = window; W.d = d; W.all = A.all; W.dmask = (1u << d) - 1u;
+    reconstruct_walk_kernel<<<wire_grid(ctx, n_groups, kWireThreads / 32), kWireThreads, 0, ctx->stream>>>(W);
+    SS_CUDA(cudaGetLastError());
+    ctx->launches++;
+
+    // reconstruct_data for the rows the walk marked; every other row reads as intact
+    return launch_rs_reconstruct_uniform(coder, shard_planes, plane_stride, shard_stride, data_len, dec_present, n, 1, dec_status);
 }
 
 }  // extern "C"
